@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA arm
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the restated mj_step on the host cores
+    python bench.py ... --dump-outputs DIR                   # + the outputs of the last timed step as DIR/*.npy
 
 One "step" = one control step of every environment of the batch (walk: 10 physics substeps of 2e-4 s): workload
 `walk_imitation 4096 envs, random policy` per GPU (BASELINE.json configs[1]).  N > 1 is configs[3]: envs sharded across ranks
@@ -75,6 +76,27 @@ class ClockSampler(threading.Thread):
             if any(s[i].lower().startswith('active') for s in self.samples):
                 reasons.append(name)
         return {'sm_mhz': sm[len(sm) // 2], 'sm_max_mhz': float(self.samples[0][2]), 'reasons': reasons, 'samples': len(sm)}
+
+
+DUMP_BUDGET = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: the arrays of the last timed step as out_dir/<name>.npy (float32, or float64 for float64 data), so that
+    two builds run with the same arguments can be compared output for output.  All arrays share the env axis 0; above
+    DUMP_BUDGET bytes a fixed, seeded sample of envs is written instead, and its indices as env_index.npy."""
+    arrays = {k: np.asarray(v.detach().cpu().numpy() if hasattr(v, 'detach') else v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    headers = 128 * (len(arrays) + 1)                                  # .npy headers, env_index.npy included
+    if sum(v.nbytes for v in arrays.values()) + headers > DUMP_BUDGET:
+        per_env = sum(v.nbytes for v in arrays.values()) // n + 8        # + its float64 entry in env_index
+        keep = np.sort(np.random.RandomState(0).choice(n, (DUMP_BUDGET - headers) // per_env, replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays['env_index'] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), v)
 
 
 def start_state(m, wl, rs):
@@ -194,8 +216,9 @@ def make_env(wl, N, local, seed, device_task=True):
     return fly_envs.flight_imitation(n_envs=N, device=local, seed=seed, device_task=device_task)
 
 
-def measure(wl, args, world, rank, local, with_exchange):
-    """-> dict of raw measurements of one workload on this rank (rank 0 aggregates)"""
+def measure(wl, args, world, rank, local, with_exchange, dump_dir=None):
+    """-> dict of raw measurements of one workload on this rank (rank 0 aggregates); with `dump_dir`, the observation rows and
+    (reward, discount, step_type) of this rank's envs after the last timed step are written there"""
     import torch
     import torch.distributed as dist
     from flybody_b200 import stepper as st
@@ -258,6 +281,9 @@ def measure(wl, args, world, rank, local, with_exchange):
         ev1.record(stream)
     sim.sync(); torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1)
+    if dump_dir:
+        obs, out = state['obs'], state['out']
+        dump_outputs(dump_dir, {'observation': obs, 'reward': out[:, 0], 'discount': out[:, 1], 'step_type': out[:, 2]})
     launches = sim.launch_count - l0
     resets = int(env.device_reset_count()) - resets0
     nefc = sim.get(st.NEFC)[:, 0].astype(np.int64); ncon = sim.get(st.NCON)[:, 0].astype(np.int64)
@@ -373,12 +399,13 @@ def line_of(wl, args, world, r):
     }
 
 
-def measure_vision(args, world, rank, local, n_envs=1024):
+def measure_vision(args, world, rank, local, n_envs=1024, dump_dir=None):
     """BASELINE.json configs[4] shape: `vision_guided_flight` (heightfield terrain contacts, two 32 x 32 x 3 eye cameras rendered on the
     device every step, wing-beat pattern generator, the task's hooks as device code: fb_task_* kind 2) + the reference's vision policy
     (VisNet + two-level controller, flybody_b200/policy_torch.py, random weights) in the loop on rank 0 (observation rows + eyes of all
     ranks gathered over NCCL, actions scattered back).  `value`: everything stays in HBM (`step_device`: torch views of the rows and the
-    eye images).  `e2e`: env.step(host actions) -> observations + eyes on the host -> policy input copied up -> actions copied down."""
+    eye images).  `e2e`: env.step(host actions) -> observations + eyes on the host -> policy input copied up -> actions copied down.
+    With `dump_dir`: the rows, (reward, discount, step_type), eyes and policy actions of this rank after the last timed step."""
     import torch
     import torch.distributed as dist
     from flybody_b200 import fly_envs
@@ -454,6 +481,8 @@ def measure_vision(args, world, rank, local, n_envs=1024):
             a = act_dev(rows, eyes)
         ev1.record(stream)
         sync()
+        if dump_dir:
+            dump_outputs(dump_dir, {'observation': rows, 'reward': out[:, 0], 'discount': out[:, 1], 'step_type': out[:, 2], 'eyes': eyes, 'action': a})
         dt_dev = maxr(ev0.elapsed_time(ev1) * 1e-3)
         launches = env._sim.launch_count - l0
         resets = int(env._sim.task_episodes().sum() - e0)
@@ -506,14 +535,15 @@ def run_ours(args, wl):
         os.environ.setdefault('NCCL_DEBUG_FILE', '/dev/stderr')      # stdout carries exactly one JSON line
         dist.init_process_group('nccl', device_id=torch.device('cuda', local))
     if args.workload == 'vision':
-        res = measure_vision(args, world, rank, local, n_envs=args.envs if args.envs != ENVS_PER_GPU else 1024)
+        res = measure_vision(args, world, rank, local, n_envs=args.envs if args.envs != ENVS_PER_GPU else 1024,
+                             dump_dir=args.dump_outputs if rank == 0 else None)
         if rank == 0:
             res.update({'steps': args.steps, 'warmup': args.warmup, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic'})
             emit(res)
         if world > 1:
             dist.barrier(); dist.destroy_process_group()
         return
-    r = measure(wl, args, world, rank, local, with_exchange=world > 1)
+    r = measure(wl, args, world, rank, local, with_exchange=world > 1, dump_dir=args.dump_outputs if rank == 0 else None)
     if rank == 0:
         line = line_of(wl, args, world, r)
         if world == 1 and not args.no_extra and args.workload == 'walk':
@@ -566,7 +596,12 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip the nested flight_imitation block')
     ap.add_argument('--preroll', type=int, default=-1, help='control steps of staggered-reset pre-roll before the warm-up (-1: one episode length; 0: standing start)')
     ap.add_argument('--workload', default='walk', choices=sorted(WORKLOADS) + ['vision'], help='walk = the headline (BASELINE configs[1]); flight = configs[2]')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="CUDA arm: write what the timed path returned in its last step (rank 0's envs) as DIR/<name>.npy, at most 64 MB; "
+                         'the inputs are seeded, so runs with the same arguments can be compared output for output')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs covers the CUDA arm only: the reference arm runs for a time budget, not a number of steps')
     args.warmup = max(args.warmup, 3)
     wl = WORKLOADS.get(args.workload, WORKLOADS['flight'])
     if args.impl == 'reference':

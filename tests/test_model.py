@@ -4,9 +4,10 @@ import os
 import re
 
 import numpy as np
-import pytest
 
 from flybody_b200.flymodel import FIELDS, c_struct_text, load_model
+
+import model_goldens
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 G = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'reference_goldens.json')))
@@ -94,11 +95,10 @@ def test_header_struct_in_sync_with_field_table():
     assert len(FIELDS) == len(set(n for n, _ in FIELDS))
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/flybody'), reason='reference checkout not present')
 def test_committed_models_reproduce_from_reference_assets():
-    from flybody_b200.compiler.compile_model import compile_variant
+    """the shipped models are what the compiler makes of the reference's fruitfly.xml (tests/golden/fruitfly_assets)"""
     for variant in ('walk', 'flight'):
-        fresh = compile_variant(variant)
+        fresh = model_goldens.compile_variant(variant)
         m = load_model(variant)
         for k in ('body_mass', 'body_inertia', 'body_pos', 'geom_pos', 'dof_invweight0', 'actuator_gainprm'):
             assert np.allclose(fresh[k], getattr(m, k), rtol=1e-12, atol=0), k

@@ -2,17 +2,17 @@
 disable_legs, joint_filter; reference fly_envs.py:100-246, fruitfly.py:204-340) compiled on demand, and the reference's walker
 contracts of tests/test_flywalker.py:36-168 (all 16 use-combinations x 4 filter settings: action <-> ctrl index maps, actuator
 dyntype / dynprm, ctrlrange of named actuators, force actuators, filterexact) checked on OUR compiled models -- the reference
-checks them on MuJoCo's compilation of the same MJCF surgery.  Needs the reference's fruitfly.xml (present in the build container;
-skipped where it is not)."""
+checks them on MuJoCo's compilation of the same MJCF surgery.  Compiled from the reference's fruitfly.xml stored under
+tests/golden/fruitfly_assets; every compilation is also checked against the stored one (tests/model_goldens.py)."""
 import numpy as np
 import pytest
 
 import __graft_entry__ as ge
 from flybody_b200 import fly_envs, stepper as st
 from flybody_b200.dm_env_shim import StepType
-from flybody_b200.flymodel import from_compiled, model_for, reference_assets_dir
+from flybody_b200.flymodel import from_compiled
 
-pytestmark = pytest.mark.skipif(reference_assets_dir() is None, reason="the reference's fruitfly.xml is not available here")
+import model_goldens
 
 JOINT_FILTER, ADHESION_FILTER = 0.0123, 0.0234                     # tests/test_flywalker.py:13-14
 USES = [(i, j, k, l) for i in range(2) for j in range(2) for k in range(2) for l in range(2)]
@@ -26,9 +26,8 @@ def emu():
 
 
 def _walker(use, flt, **kw):
-    from flybody_b200.compiler import compile_model as cm
-    return from_compiled(cm.compile_variant('walker', use_legs=bool(use[0]), use_wings=bool(use[1]), use_mouth=bool(use[2]),
-                                            use_antennae=bool(use[3]), joint_filter=flt[0], adhesion_filter=flt[1], **kw))
+    return from_compiled(model_goldens.compile_variant('walker', use_legs=bool(use[0]), use_wings=bool(use[1]), use_mouth=bool(use[2]),
+                                                       use_antennae=bool(use[3]), joint_filter=flt[0], adhesion_filter=flt[1], **kw))
 
 
 def test_fly_bulletproof_contracts_on_the_compiled_walker(emu):
@@ -77,6 +76,7 @@ def test_force_actuators_and_filterexact():
 def test_env_factories_accept_the_reference_switches(emu, tmp_path, monkeypatch):
     """walk_imitation(force_actuators / disable_wings=False / joint_filter) and flight_imitation(disable_legs=False / joint_filter):
     compiled on first use, cached, stepped; the flight env with legs gains the leg observables (tasks/base.py:360-364)."""
+    monkeypatch.setenv('FLYBODY_ASSETS', model_goldens.ASSETS)
     monkeypatch.setenv('FLYBODY_B200_CACHE', str(tmp_path))
     env = fly_envs.walk_imitation(n_envs=2, lib_path=emu, disable_wings=False, terminal_com_dist=float('inf'))
     assert env.action_spec().shape == (65,) and 'wing_yaw_left' in env.action_spec().name
@@ -104,3 +104,8 @@ def test_env_factories_accept_the_reference_switches(emu, tmp_path, monkeypatch)
     env.reset(); ts = env.step(np.zeros((2, 65), np.float32))
     assert np.all(ts.reward == 1)
     env.close()
+    # the cached compilations against the stored ones (the switches as model_for hands them to the compiler)
+    sw = dict(force_actuators=False, use_wings=None, use_legs=None, joint_filter=None)
+    for name, variant, kw in (('fly_walk_wings', 'walk', dict(sw, use_wings=True)), ('fly_walk_force_jf0', 'walk', dict(sw, force_actuators=True, joint_filter=0.0)),
+                              ('fly_flight_legs_jf0.0002', 'flight', dict(sw, use_legs=True, joint_filter=0.0002))):
+        model_goldens.assert_matches_stored(*model_goldens.read_saved(str(tmp_path / f'{name}.npz')), variant, **kw)
